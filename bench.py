@@ -2,6 +2,7 @@
 """bench.py — images/sec of the txt2img hot path (CFG denoising loop + VAE decode), the metric BASELINE.json names.
 
   python bench.py --gpus N --steps K --warmup W [--config sd15|sdxl] [--dtype bf16|fp16] [--impl sdxe|reference] [--only-headline]
+                   [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch: `process_images` of B images. ONE invocation measures the whole
 metric and prints ONE JSON line:
@@ -37,6 +38,7 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 # algorithmic work (BASELINE.md §2 / SURVEY §8(d)): 2*MAC over conv / linear / QK^T / PV, no padding, no recompute
@@ -298,9 +300,20 @@ def class_table(prof):
                 "gbs": (v["bytes"] / (v["ms"] / 1e3) / 1e9 if v["ms"] > 0 else 0), "launches": v["launches"]} for k, v in prof.items()}
 
 
-def measure_workload(key, dtype_name, rank, world, local, device, steps, warmup, want_roofline, want_extras, want_parity, clock_sampler=None):
+def dump_outputs(dump_dir, outputs):
+    """Writes each array as DIR/<name>.npy in float32 (uint8 pixels convert exactly). The largest workload's images
+    (SDXL or hires fix, 4 x 1024 x 1024 x 3) come to 48 MiB, so every output is stored whole."""
+    os.makedirs(dump_dir, exist_ok=True)
+    for name, t in outputs.items():
+        np.save(os.path.join(dump_dir, f"{name}.npy"), t.float().numpy())
+
+
+def measure_workload(key, dtype_name, rank, world, local, device, steps, warmup, want_roofline, want_extras, want_parity, clock_sampler=None,
+                     dump_dir=None):
     """Builds the model, runs W warm-ups, times K resident steps and K end-to-end steps (max over ranks, barrier + device
-    sync on both sides), optionally the roofline pass / baselines / shard-parity check. Returns the JSON block (rank 0) or None."""
+    sync on both sides), optionally the roofline pass / baselines / shard-parity check. Returns the JSON block (rank 0) or None.
+    With `dump_dir`, rank 0 writes what the last timed resident step returned for its own shard: `images` [B, H, W, 3]
+    and `latents` [B, 4, h, w]."""
     import torch.distributed as dist
 
     from sdwebui_b200 import lib as L
@@ -342,7 +355,7 @@ def measure_workload(key, dtype_name, rank, world, local, device, steps, warmup,
         n0 = lib.sdxe_launch_count()
         e0.record()
         for _ in range(k):
-            fn()
+            out = fn()
         e1.record()
         barrier()
         ms = e0.elapsed_time(e1)
@@ -350,7 +363,7 @@ def measure_workload(key, dtype_name, rank, world, local, device, steps, warmup,
             tms = torch.tensor([ms], device=device)
             dist.all_reduce(tms, op=dist.ReduceOp.MAX)
             ms = tms.item()
-        return ms, lib.sdxe_launch_count() - n0
+        return ms, lib.sdxe_launch_count() - n0, out
 
     for _ in range(warmup):
         step_resident()
@@ -366,9 +379,13 @@ def measure_workload(key, dtype_name, rank, world, local, device, steps, warmup,
         n_roll += 1
     if clock_sampler is not None:
         clock_sampler.start()
-    ms_res, launches = timed(step_resident, steps)
-    ms_e2e, _ = timed(step_e2e, steps)
+    ms_res, launches, last = timed(step_resident, steps)
+    # copied to the host before the next timed region can reuse the device buffers
+    outputs = {"images": last.images.cpu(), "latents": last.latents.cpu()} if dump_dir and rank == 0 else None
+    ms_e2e, _, _ = timed(step_e2e, steps)
     clocks = clock_sampler.stop() if clock_sampler is not None else None
+    if outputs is not None:
+        dump_outputs(dump_dir, outputs)
 
     # ---- shard parity: rank 0 regenerates the LAST rank's images (N = 1: its own, a second time) and compares pixels
     parity = None
@@ -474,7 +491,14 @@ def main():
     ap.add_argument("--dtype", default="bf16", choices=["bf16", "fp16"])
     ap.add_argument("--no-extras", action="store_true", help="skip cpu_baseline / torch-SDP legs")
     ap.add_argument("--only-headline", action="store_true", help="skip the fp16 / sdxl / c4 blocks")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the headline's last timed step returned as DIR/<name>.npy (float32); "
+                         "weights, conditioning and noise are seeded, so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the sdxe path's outputs; the reference arm only times a CPU sample")
 
     from sdwebui_b200 import parallel as P
 
@@ -493,7 +517,8 @@ def main():
     extras = not args.no_extras
     warm = max(3, args.warmup)
     sampler = ClockSampler(local) if rank == 0 else None
-    head = measure_workload(args.config, args.dtype, rank, world, local, device, args.steps, warm, True, extras, True, sampler)
+    head = measure_workload(args.config, args.dtype, rank, world, local, device, args.steps, warm, True, extras, True, sampler,
+                            args.dump_outputs)
     blocks = {}
     if not args.only_headline:
         sub_steps = max(1, min(args.steps, 5))
